@@ -2,6 +2,7 @@
 """bench.py -- fwd+bwd Mpixels/s of the rasterise hot path on BASELINE.json's workload.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg3|cfg4|cfg5|cfg2|cube]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one forward + one backward pass of the hot path over one batch of synthetic scenes
@@ -19,6 +20,8 @@ One JSON line on rank 0:  value = B_total*H*W / step time (CUDA events, max over
 call with HOST (pinned) buffers, host<->device copies inside the timed region;  roofline = the dominant
 kernel against the measured HBM copy peak;  cpu_baseline = the CPU oracle on a bounded sample.
 --impl reference times the CPU port of the reference path (oracle/), the only runnable reference here.
+--dump-outputs DIR writes the outputs of the last timed step as .npy files (dump_outputs); the inputs are seeded, so two
+builds run with the same arguments can be compared output for output.  The bench writes nothing into the tree.
 """
 import argparse
 import ctypes
@@ -33,6 +36,7 @@ import numpy as np
 
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True   # the tree may be read-only: no __pycache__ is written next to the sources
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
@@ -417,6 +421,34 @@ def check_against_oracle(prep, scene, images=1):
     return res
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(prep, which, out_dir, seed=0):
+    """Writes what a caller of the timed path receives from its last step (gradient buffer `which`) as out_dir/<name>.npy:
+    the batch-accumulated grad_vertices [V,4] and grad_vertex_colors [V,C] (summed over the ranks when N > 1), and
+    pixels [n,C], face_ids [n] and grad_background [n,C] at the n pixels listed in pixel_index [n] (flat index b*H*W + y*W + x).
+    n is every pixel of the batch, or a fixed sample drawn with `seed` when that would exceed DUMP_BYTES in all, so two builds
+    run with the same arguments can be compared file for file."""
+    torch = prep.torch
+    B, H, W, C, V, F = prep.dims
+    flat = prep.reduced_flat[which] if prep.peer is not None else prep.shared_flat[which]
+    out = {'grad_vertices': flat[:V * 4].view(V, 4).cpu().numpy(),
+           'grad_vertex_colors': flat[V * 4:V * (4 + C)].view(V, C).cpu().numpy()}
+    n_pix = B * H * W
+    per_pixel = 4 * (2 * C + 1) + 8   # pixels and grad_background (C float32 each), the face id (float32), the index (float64)
+    n = min(n_pix, (DUMP_BYTES - 4096 - sum(a.nbytes for a in out.values())) // per_pixel)   # 4096: the six .npy headers
+    index = np.arange(n_pix) if n == n_pix else np.sort(np.random.default_rng(seed).choice(n_pix, size=n, replace=False))
+    idx = torch.from_numpy(index).to(prep.device)
+    out['pixel_index'] = index.astype(np.float64)
+    out['pixels'] = prep.pixels.view(n_pix, C)[idx].cpu().numpy()
+    out['face_ids'] = prep.face_ids.view(n_pix)[idx].float().cpu().numpy()   # exact: face ids stay below 2^24
+    out['grad_background'] = prep.grad_background.view(n_pix, C)[idx].cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + '.npy'), a)
+
+
 def numpy_baselines(scene, grad_pixels, threads, one_process_images=2, budget_s=20.0):
     """The reference-style numpy path (oracle/numpy_raster.py: coverage on a meshgrid of pixel centres, as
     tests/square_test.py:11-17 does for its square) fwd+bwd: (i) one process, (ii) a multiprocessing pool over the
@@ -491,8 +523,8 @@ def run_ours(args):
         import torch.distributed as dist
         dist.init_process_group('nccl', device_id=device, timeout=datetime.timedelta(seconds=120))
     from dirt_b200 import build as lib_build, scenes
-    if rank == 0:
-        lib_build.build()
+    if rank == 0 and lib_build.is_stale():   # the bench times the library build() made; it never compiles into the tree
+        sys.stderr.write('bench: %s is missing or older than its sources: run build() first\n' % lib_build.SO_PATH)
     if world > 1:
         dist.barrier()
 
@@ -548,6 +580,8 @@ def run_ours(args):
     stop.record()
     sync_all()
     elapsed_ms = start.elapsed_time(stop)
+    if args.dump_outputs and rank == 0:   # before anything below overwrites the buffers of the last timed step
+        dump_outputs(prep, prep.parity ^ 1, args.dump_outputs)
     # keep the GPU busy a little longer so the clock sampler sees the loaded state even for short runs
     if sampler:   # rank 0 only: no collectives in here
         t_end = time.time() + 0.6
@@ -837,7 +871,13 @@ def main():
                     help='after timing, validate the benched buffers against the CPU oracle ("checked": true); on by default')
     ap.add_argument('--no-check', dest='check', action='store_false', help='skip that validation')
     ap.add_argument('--no-numa-bind', action='store_true', help='do not pin the process to the NUMA node of its GPU')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='after the timed steps, write what the last one computed to DIR/<name>.npy '
+                                                           '(float32/float64, at most 64 MB: a fixed sample of the pixels)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs needs --impl ours')
     if args.impl == 'reference':
         run_reference(args)
     else:

@@ -9,6 +9,7 @@ the OpenGL driver renders in the reference) is an input -- tests feed it the CPU
 Only tests/, tests/golden/make_ref_golden.py and __graft_entry__.build() may use this module.
 """
 import ctypes
+import hashlib
 import os
 import subprocess
 
@@ -51,6 +52,17 @@ def lib():
 
 def _f32(a):
     return np.ascontiguousarray(a, dtype=np.float32)
+
+
+def fingerprint(*arrays):
+    """sha256 over the dtype, shape and bytes of each array.  Golden data records with it, bit for bit, inputs and outputs
+    of a reference-kernel run that are too large to store (tests/golden/ref_live_scenes.npz)."""
+    h = hashlib.sha256()
+    for a in arrays:
+        a = np.ascontiguousarray(a)
+        h.update(('%s%s' % (a.dtype.str, a.shape)).encode())
+        h.update(a.tobytes())
+    return h.hexdigest()
 
 
 def _ptr(a):
