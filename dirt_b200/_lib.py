@@ -22,6 +22,9 @@ ERR_STALE_WORKSPACE = -8
 BWD_SHARED_GEOMETRY = 1
 BWD_SKIP_POSITION = 2
 BWD_SKIP_COLOUR = 4
+SHARED_BACKGROUND = 8
+SHARED_COLOURS = 16
+SHARED_FACES = 32
 
 
 def lib():
@@ -46,6 +49,8 @@ def lib():
     L.dirt_workspace_bytes_min.argtypes = [i] * 6
     L.dirt_rasterise_forward.restype = i
     L.dirt_rasterise_forward.argtypes = [vp] * 6 + [i] * 6 + [vp, sz, vp]
+    L.dirt_rasterise_forward_ex.restype = i
+    L.dirt_rasterise_forward_ex.argtypes = [vp] * 6 + [i] * 6 + [vp, sz, vp, i]
     L.dirt_rasterise_backward.restype = i
     L.dirt_rasterise_backward.argtypes = [vp] * 8 + [i] * 6 + [ctypes.POINTER(ctypes.c_int), i, i, vp, sz, vp]
     L.dirt_rasterise_backward_ex.restype = i
@@ -66,6 +71,7 @@ def lib():
 
 
 EXPORTED_SYMBOLS = ['dirt_error_string', 'dirt_abi_version', 'dirt_workspace_bytes', 'dirt_workspace_bytes_min', 'dirt_rasterise_forward',
+                    'dirt_rasterise_forward_ex',
                     'dirt_rasterise_backward', 'dirt_rasterise_backward_ex', 'dirt_workspace_status',
                     'dirt_rasterise_visibility', 'dirt_peer_exchange_bytes', 'dirt_peer_exchange', 'dirt_last_launch_count',
                     'dirt_kernel_timer_enable', 'dirt_kernel_timer_elapsed_ms']

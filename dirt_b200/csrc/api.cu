@@ -7,7 +7,11 @@
 using namespace dirt;
 
 static_assert(BWD_SHARED_GEOMETRY == DIRT_BWD_SHARED_GEOMETRY && BWD_SKIP_POSITION == DIRT_BWD_SKIP_POSITION &&
-              BWD_SKIP_COLOUR == DIRT_BWD_SKIP_COLOUR, "flag values of common.cuh and dirt_b200.h differ");
+              BWD_SKIP_COLOUR == DIRT_BWD_SKIP_COLOUR && SHARED_BACKGROUND == DIRT_SHARED_BACKGROUND &&
+              SHARED_COLOURS == DIRT_SHARED_COLOURS && SHARED_FACES == DIRT_SHARED_FACES,
+              "flag values of common.cuh and dirt_b200.h differ");
+
+static constexpr int SHARING_BITS = DIRT_SHARED_BACKGROUND | DIRT_SHARED_COLOURS | DIRT_SHARED_FACES;
 
 static thread_local int t_last_launches = 0;
 
@@ -42,7 +46,7 @@ KernelTimer& kernel_timer()
 extern "C" int dirt_kernel_timer_enable(int which)
 {
     KernelTimer& t = kernel_timer();
-    if (which < 0 || which > 2) return DIRT_ERR_BAD_SHAPE;
+    if (which < 0 || which > 3) return DIRT_ERR_BAD_SHAPE;
     if (which != 0 && !t.start) {
         if (cudaEventCreate(&t.start) != cudaSuccess || cudaEventCreate(&t.stop) != cudaSuccess) {
             t.start = t.stop = nullptr;
@@ -135,13 +139,14 @@ static int check_workspace(void* workspace, size_t workspace_bytes, int B, int H
         if (e__ != cudaSuccess) { t_last_launches = launches; return DIRT_ERR_CUDA; } \
     } while (0)
 
-extern "C" int dirt_rasterise_forward(const float* background, const float* vertices, const float* vertex_colors,
-                                      const int32_t* faces, float* pixels, int32_t* face_ids_out, int B, int H, int W,
-                                      int C, int V, int F, void* workspace, size_t workspace_bytes, void* cuda_stream)
+extern "C" int dirt_rasterise_forward_ex(const float* background, const float* vertices, const float* vertex_colors,
+                                         const int32_t* faces, float* pixels, int32_t* face_ids_out, int B, int H, int W,
+                                         int C, int V, int F, void* workspace, size_t workspace_bytes, void* cuda_stream, int flags)
 {
     int launches = 0;
     t_last_launches = 0;
     if (!shape_ok(B, H, W, C, V, F)) return DIRT_ERR_BAD_SHAPE;
+    if (flags & ~SHARING_BITS) return DIRT_ERR_BAD_SHAPE;
     if (B == 0) return DIRT_OK;
     if (!background || !pixels) return DIRT_ERR_NULL_POINTER;
     if ((V > 0 && (!vertices || !vertex_colors)) || (F > 0 && !faces)) return DIRT_ERR_NULL_POINTER;
@@ -153,11 +158,19 @@ extern "C" int dirt_rasterise_forward(const float* background, const float* vert
     if (rc != DIRT_OK) return rc;
     cudaStream_t stream = (cudaStream_t)cuda_stream;
     const Workspace ws = carve_workspace(workspace, B, H, W, C, V, F);
-    const Dims d = make_dims(B, H, W, C, V, F);
+    const Dims d = make_dims(B, H, W, C, V, F, flags);
     CUDA_TRY(launch_setup_and_bin(vertices, faces, vertex_colors, ws, d, stream, &launches));
     CUDA_TRY(launch_raster_forward(vertices, background, vertex_colors, pixels, face_ids_out, ws, d, stream, &launches));
     t_last_launches = launches;
     return DIRT_OK;
+}
+
+extern "C" int dirt_rasterise_forward(const float* background, const float* vertices, const float* vertex_colors,
+                                      const int32_t* faces, float* pixels, int32_t* face_ids_out, int B, int H, int W,
+                                      int C, int V, int F, void* workspace, size_t workspace_bytes, void* cuda_stream)
+{
+    return dirt_rasterise_forward_ex(background, vertices, vertex_colors, faces, pixels, face_ids_out, B, H, W, C, V, F,
+                                     workspace, workspace_bytes, cuda_stream, 0);
 }
 
 extern "C" int dirt_rasterise_visibility(const float* vertices, const int32_t* faces, int32_t* face_ids, float* gbuffer,
@@ -191,14 +204,15 @@ static int backward_impl(const float* vertices, const int32_t* faces, const floa
     t_last_launches = 0;
     if (!shape_ok(B, H, W, C, V, F)) return DIRT_ERR_BAD_SHAPE;
     if (V > (1 << 24)) return DIRT_ERR_TOO_MANY_VERTICES;
-    if (flags & ~(DIRT_BWD_SHARED_GEOMETRY | DIRT_BWD_SKIP_POSITION | DIRT_BWD_SKIP_COLOUR)) return DIRT_ERR_BAD_SHAPE;
+    if (flags & ~(DIRT_BWD_SHARED_GEOMETRY | DIRT_BWD_SKIP_POSITION | DIRT_BWD_SKIP_COLOUR | SHARING_BITS)) return DIRT_ERR_BAD_SHAPE;
     GroupSpec groups;
     int rc = make_groups(C, channel_groups, n_groups, &groups);
     if (rc != DIRT_OK) return rc;
     if (B == 0) return DIRT_OK;
     if (!grad_pixels) return DIRT_ERR_NULL_POINTER;
     if (!(flags & DIRT_BWD_SKIP_POSITION) && !pixels) return DIRT_ERR_NULL_POINTER;
-    if (!(flags & DIRT_BWD_SKIP_COLOUR) && !grad_background) return DIRT_ERR_NULL_POINTER;
+    // a shared background's gradient may be NULL: not wanted
+    if (!(flags & (DIRT_BWD_SKIP_COLOUR | DIRT_SHARED_BACKGROUND)) && !grad_background) return DIRT_ERR_NULL_POINTER;
     if ((V > 0 && (!vertices || !grad_vertices || !grad_vertex_colors)) || (F > 0 && !faces)) return DIRT_ERR_NULL_POINTER;
     if ((uintptr_t)vertices % 16 != 0 || (uintptr_t)grad_vertices % 16 != 0) return DIRT_ERR_MISALIGNED;
     if ((uintptr_t)pixels % 4 || (uintptr_t)grad_pixels % 4 || (uintptr_t)grad_background % 4 ||
@@ -208,7 +222,7 @@ static int backward_impl(const float* vertices, const int32_t* faces, const floa
     if (rc != DIRT_OK) return rc;
     cudaStream_t stream = (cudaStream_t)cuda_stream;
     const Workspace ws = carve_workspace(workspace, B, H, W, C, V, F);
-    const Dims d = make_dims(B, H, W, C, V, F);
+    const Dims d = make_dims(B, H, W, C, V, F, flags & SHARING_BITS);
     const int32_t* ids = face_ids;
     // the tile coverage flags in the workspace describe `ids` when the raster kernel that produced them ran on this workspace
     const bool flags_valid = !ids || workspace_holds_setup;
@@ -222,7 +236,7 @@ static int backward_impl(const float* vertices, const int32_t* faces, const floa
         CUDA_TRY(launch_setup_only(vertices, faces, ws, d, stream, &launches));
     } else {
         // a promise: checked on the device against the tag the setup pass left in the workspace
-        expect_tag = workspace_tag(vertices, faces, B, H, W, V, F);
+        expect_tag = workspace_tag(vertices, faces, B, H, W, V, F, d.face_stride == 0);
     }
     CUDA_TRY(launch_backward(vertices, pixels, grad_pixels, ids, grad_background, grad_vertices, grad_vertex_colors, ws, d,
                              groups, flags_valid, flags, expect_tag, stream, &launches));

@@ -35,6 +35,7 @@
 
 #include <cuda.h>
 #include <cudaTypedefs.h>
+#include <type_traits>
 
 namespace dirt {
 
@@ -483,7 +484,8 @@ __global__ void __launch_bounds__(NW * 32, DIRT_BWD_MIN_BLOCKS * DIRT_BWD_WARPS 
     float* __restrict__ grad_vertex_colors, Workspace ws, Dims d, const unsigned char* __restrict__ tile_flags,
     int cs, int c0,   // cs: channels per pixel in the tensors, c0: first channel of the group this launch handles (width C)
     int gstride,      // floats per vertex row of grad_vertex_colors as this launch sees it (cs, or 4 for the padded rows of C = 3)
-    int flags,        // BWD_SHARED_GEOMETRY: vertex gradients accumulated over the batch ([V,.]); BWD_SKIP_POSITION / _COLOUR
+    int flags,        // BWD_SHARED_GEOMETRY: vertex gradients accumulated over the batch ([V,.]); BWD_SKIP_POSITION / _COLOUR;
+                      // SHARED_COLOURS: grad_vertex_colors accumulated over the batch; SHARED_BACKGROUND: no grad_background here
     unsigned long long expect_tag,   // != 0: the caller promised that the workspace holds the setup records with this tag
     int b_base)                      // first image of this launch (the grid's z extent holds at most 65535 images)
 {
@@ -508,6 +510,7 @@ __global__ void __launch_bounds__(NW * 32, DIRT_BWD_MIN_BLOCKS * DIRT_BWD_WARPS 
     const int lcol = lane & 7, lrow0 = (lane >> 3) * 2;
     const int row0 = trow0 + lrow0, col = tcol0 + lcol;
     const bool want_pos = !(flags & BWD_SKIP_POSITION), want_col = !(flags & BWD_SKIP_COLOUR);
+    const bool write_gb = want_col && !(flags & SHARED_BACKGROUND);   // the per-image grad_background
 
     if (expect_tag != 0 && (blockIdx.x | blockIdx.y | (unsigned)b | threadIdx.x) == 0 && ws.header->tag != expect_tag) {
         // the workspace was not filled by a forward / visibility call on these (vertices, faces, sizes): flag it
@@ -524,6 +527,7 @@ __global__ void __launch_bounds__(NW * 32, DIRT_BWD_MIN_BLOCKS * DIRT_BWD_WARPS 
         if (lane == 0) f = tile_flags == nullptr || tile_flags[(size_t)b * d.tiles + ty * d.tiles_x + (tx >> 1)] != 0;
         flagged = (__ballot_sync(0xffffffffu, f) & 1u) != 0u;   // through a vote: known to be warp-uniform
     }
+    if (!flagged && !write_gb) return;   // no face can reach the tile and no grad_background to write: grad_pixels is not read
     const size_t img = (size_t)b * H * W;
     const size_t p0 = img + (size_t)row0 * W + col;   // pixel 0 of this lane (pixel 1: + W)
     const bool in0 = col < W && row0 < H, in1 = col < W && row0 + 1 < H;
@@ -555,8 +559,8 @@ __global__ void __launch_bounds__(NW * 32, DIRT_BWD_MIN_BLOCKS * DIRT_BWD_WARPS 
     };
     if (!flagged) {
         // the forward pass flagged every 16x8 tile that shows a face or touches one that does: nothing can reach this one
-        if (want_col && in0) store_gb(0, true);
-        if (want_col && in1) store_gb(1, true);
+        if (in0) store_gb(0, true);
+        if (in1) store_gb(1, true);
         return;
     }
 
@@ -580,7 +584,7 @@ __global__ void __launch_bounds__(NW * 32, DIRT_BWD_MIN_BLOCKS * DIRT_BWD_WARPS 
     const TriInterp* itp_b = ws.itp + (size_t)b * d.F;
     const TriXY* xy_b = ws.xy + (size_t)b * d.F;
     float* gverts = grad_vertices + (size_t)(per_item ? b : 0) * d.V * 4;
-    float* gcols = grad_vertex_colors + (size_t)(per_item ? b : 0) * d.V * gstride + c0;
+    float* gcols = grad_vertex_colors + (size_t)(per_item && !(flags & SHARED_COLOURS) ? b : 0) * d.V * gstride + c0;
 
     // ---- (1) stage the halo of face ids and pixels: TMA (one elected lane, one mbarrier each) or per-lane cp.async
     if (use_tma) {
@@ -623,8 +627,8 @@ __global__ void __launch_bounds__(NW * 32, DIRT_BWD_MIN_BLOCKS * DIRT_BWD_WARPS 
     __syncwarp();
     const int i0 = (lrow0 + 1) * IDS_COLS + lcol + 1 + IDS_COL0;
     const int id0 = ids_tile[i0], id1 = ids_tile[i0 + IDS_COLS], idr = ids_tile[ring_r * IDS_COLS + ring_c + IDS_COL0];
-    if (want_col && in0) store_gb(0, id0 < 0);
-    if (want_col && in1) store_gb(1, id1 < 0);
+    if (write_gb && in0) store_gb(0, id0 < 0);
+    if (write_gb && in1) store_gb(1, id1 < 0);
     // neighbours in the visibility buffer
     const int up0 = ids_tile[i0 - IDS_COLS], l0 = ids_tile[i0 - 1], r0 = ids_tile[i0 + 1];
     const int l1 = ids_tile[i0 + IDS_COLS - 1], r1 = ids_tile[i0 + IDS_COLS + 1], dn1 = ids_tile[i0 + 2 * IDS_COLS];
@@ -942,6 +946,42 @@ __global__ void __launch_bounds__(256) unpad_rows_kernel(const float* __restrict
     out[i] = in[r * 4 + (i - r * 3)];
 }
 
+// grad_background of a background the batch shares: grad_bg[h,w,c] = sum_b [face_ids[b,h,w] < 0] * grad_pixels[b,h,w,c], the
+// batch sum of what the tile kernel writes per image (store_gb; assemble_grads :143-148).  One thread per pixel (VEC4: C = 4,
+// one 16-byte load per image) or per element; the sum runs in fp32 in increasing b without atomics, so the result is
+// deterministic and equal, bit for bit, to a sequential fp32 loop over the per-image gradients.  UNROLL images' loads are
+// issued before any of them is added.
+__device__ __forceinline__ void add_to(float& a, float v) { a += v; }
+__device__ __forceinline__ void add_to(float4& a, float4 v) { a.x += v.x; a.y += v.y; a.z += v.z; a.w += v.w; }
+
+template <bool VEC4>
+__global__ void __launch_bounds__(256) background_grad_kernel(const float* __restrict__ grad_pixels, const int32_t* __restrict__ face_ids,
+                                                             float* __restrict__ grad_background, int B, long long HW, int C)
+{
+    using T = typename std::conditional<VEC4, float4, float>::type;
+    constexpr int UNROLL = 8;
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;   // pixel (VEC4) or element of [H,W,C]
+    const long long img = VEC4 ? HW : HW * C;                              // T elements per image
+    if (i >= img) return;
+    const long long pix = VEC4 ? i : i / C;
+    const T* gp = reinterpret_cast<const T*>(grad_pixels) + i;
+    T acc{};
+    for (int b0 = 0; b0 < B; b0 += UNROLL) {
+        int id[UNROLL];
+        T v[UNROLL];
+#pragma unroll
+        for (int k = 0; k < UNROLL; ++k) {
+            id[k] = 0;
+            v[k] = T{};
+            if (b0 + k < B) { id[k] = __ldg(face_ids + (b0 + k) * HW + pix); v[k] = __ldg(gp + (b0 + k) * img); }
+        }
+#pragma unroll
+        for (int k = 0; k < UNROLL; ++k)
+            if (id[k] < 0) add_to(acc, v[k]);   // covered pixels (and images past the batch) add nothing
+    }
+    reinterpret_cast<T*>(grad_background)[i] = acc;
+}
+
 // ---- host side --------------------------------------------------------------------------------------------------------
 static PFN_cuTensorMapEncodeTiled tensor_map_encoder()
 {
@@ -1000,26 +1040,38 @@ cudaError_t launch_backward(const float* vertices, const float* pixels, const fl
                             bool tile_flags_valid, int flags, unsigned long long expect_tag, cudaStream_t stream, int* launches)
 {
     cudaError_t e;
-    const size_t rows = (size_t)((flags & BWD_SHARED_GEOMETRY) ? 1 : d.B) * d.V;
+    const size_t vrows = (size_t)((flags & BWD_SHARED_GEOMETRY) ? 1 : d.B) * d.V;                      // rows of grad_vertices
+    const size_t crows = (size_t)((flags & (BWD_SHARED_GEOMETRY | SHARED_COLOURS)) ? 1 : d.B) * d.V;  // rows of grad_vertex_colors
     // C = 3 as one group: colour gradients go to padded rows in the workspace (see unpad_rows_kernel)
-    const bool padded = d.C == 3 && groups.n == 1 && ws.gc_pad != nullptr && rows > 0;
+    const bool padded = d.C == 3 && groups.n == 1 && ws.gc_pad != nullptr && crows > 0;
     float* const gc_out = grad_vertex_colors;
     if (padded) grad_vertex_colors = ws.gc_pad;
     const int gstride = padded ? 4 : d.C;
-    if (grad_vertex_colors == grad_vertices + rows * 4) {
+    if (grad_vertex_colors == grad_vertices + vrows * 4) {
         // the two gradients are the halves of one flat buffer (what a multi-GPU job exchanges): one memset node
-        if ((e = cudaMemsetAsync(grad_vertices, 0, sizeof(float) * rows * (4 + gstride), stream)) != cudaSuccess) return e;
+        if ((e = cudaMemsetAsync(grad_vertices, 0, sizeof(float) * (vrows * 4 + crows * gstride), stream)) != cudaSuccess) return e;
     } else {
-        if ((e = cudaMemsetAsync(grad_vertices, 0, sizeof(float) * rows * 4, stream)) != cudaSuccess) return e;
-        if ((e = cudaMemsetAsync(grad_vertex_colors, 0, sizeof(float) * rows * gstride, stream)) != cudaSuccess) return e;
+        if ((e = cudaMemsetAsync(grad_vertices, 0, sizeof(float) * vrows * 4, stream)) != cudaSuccess) return e;
+        if ((e = cudaMemsetAsync(grad_vertex_colors, 0, sizeof(float) * crows * gstride, stream)) != cudaSuccess) return e;
     }
     const auto finish = [&]() -> cudaError_t {
         if (!padded) return cudaSuccess;
-        const long long n = (long long)rows * 3;
-        unpad_rows_kernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(grad_vertex_colors, gc_out, (long long)rows);
+        const long long n = (long long)crows * 3;
+        unpad_rows_kernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(grad_vertex_colors, gc_out, (long long)crows);
         ++*launches;
         return cudaGetLastError();
     };
+    if ((flags & SHARED_BACKGROUND) && !(flags & BWD_SKIP_COLOUR) && grad_background && d.B > 0) {
+        // the batch-summed gradient of a shared background: one launch per call, whatever the channel grouping
+        ScopedKernelTimer timer(3, stream);
+        const long long HW = (long long)d.H * d.W;
+        const bool vec4 = d.C == 4 && (((uintptr_t)grad_pixels | (uintptr_t)grad_background) % 16 == 0);
+        const long long n = vec4 ? HW : HW * d.C;
+        if (vec4) background_grad_kernel<true><<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(grad_pixels, face_ids, grad_background, d.B, HW, d.C);
+        else background_grad_kernel<false><<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(grad_pixels, face_ids, grad_background, d.B, HW, d.C);
+        ++*launches;
+        if ((e = cudaGetLastError()) != cudaSuccess) return e;
+    }
     const long long total_tiles = (long long)d.B * d.btiles;
     if (total_tiles == 0) return finish();
     ScopedKernelTimer timer(2, stream);

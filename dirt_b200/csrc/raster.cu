@@ -311,23 +311,25 @@ __global__ void __launch_bounds__(WARPS_PER_BLOCK * 32, DIRT_RASTER_MIN_BLOCKS) 
         const int cnt_a = cp[0], cnt_b = cp[1];
         if (cnt_a == 0 && cnt_b == 0 && ws.large_count[b] == 0) {
             const int col0 = txb * TILE_W + (lane & 7) * 2, row0 = trow0 + (lane >> 3) * 2;
-            const size_t p00 = ((size_t)b * d.H + row0) * d.W + col0;
+            const size_t l00 = (size_t)row0 * d.W + col0;   // pixel (row0, col0) inside the image
+            const size_t p00 = (size_t)b * d.H * d.W + l00;  // ... and in the batch
+            const size_t bg00 = (size_t)b * d.bg_stride + l00;   // ... and in the background
             if (CT == 4) {
-                const float4* src = reinterpret_cast<const float4*>(background);
+                const float4* src = reinterpret_cast<const float4*>(background) + bg00;
                 float4* dst = reinterpret_cast<float4*>(pixels);
                 float4 v[8];
 #pragma unroll
-                for (int i = 0; i < 8; ++i) v[i] = __ldg(src + p00 + (size_t)((i >> 1) & 1) * d.W + (i & 1) + (i >> 2) * TILE_W);
+                for (int i = 0; i < 8; ++i) v[i] = __ldg(src + (size_t)((i >> 1) & 1) * d.W + (i & 1) + (i >> 2) * TILE_W);
 #pragma unroll
                 for (int i = 0; i < 8; ++i) dst[p00 + (size_t)((i >> 1) & 1) * d.W + (i & 1) + (i >> 2) * TILE_W] = v[i];
             } else {
                 // CT == 3: the two pixels of a quad row are 24 contiguous, 8-byte aligned bytes (checked at launch)
-                const float2* src = reinterpret_cast<const float2*>(background);
+                const float2* src = reinterpret_cast<const float2*>(background + bg00 * 3);
                 float2* dst = reinterpret_cast<float2*>(pixels);
                 float2 v[12];
 #pragma unroll
                 for (int i = 0; i < 4; ++i) {   // i: bit 0 = row of the quad, bit 1 = tile of the pair
-                    const size_t q = (p00 + (size_t)(i & 1) * d.W + (i >> 1) * TILE_W) * 3 / 2;
+                    const size_t q = ((size_t)(i & 1) * d.W + (i >> 1) * TILE_W) * 3 / 2;
                     v[3 * i] = __ldg(src + q); v[3 * i + 1] = __ldg(src + q + 1); v[3 * i + 2] = __ldg(src + q + 2);
                 }
 #pragma unroll
@@ -356,7 +358,7 @@ __global__ void __launch_bounds__(WARPS_PER_BLOCK * 32, DIRT_RASTER_MIN_BLOCKS) 
     if (MODE == 0 && CT == 4 && lane < 16) {
         const int r = trow0 + (lane >> 1), c = tcol0 + (lane & 1) * 8;
         if (r < d.H && c < d.W)
-            asm volatile("prefetch.global.L2 [%0];" ::"l"(background + (((size_t)b * d.H + r) * d.W + c) * 4));
+            asm volatile("prefetch.global.L2 [%0];" ::"l"(background + ((size_t)b * d.bg_stride + (size_t)r * d.W + c) * 4));
     }
 #endif
     const int nbin = ws.tile_count[(size_t)b * d.tiles + t];
@@ -368,13 +370,16 @@ __global__ void __launch_bounds__(WARPS_PER_BLOCK * 32, DIRT_RASTER_MIN_BLOCKS) 
 
     // ---- nothing binned to this tile: the background passes through ----------------------------------------
     if (nbin == 0 && nlarge == 0) {
+        // pixel (row0, col0) of the background: p00 less the images a shared background does not have (a 32 x 32 -> 64-bit
+        // product: this form keeps the kernel's register allocation as it was without shared backgrounds)
+        const size_t l00 = p00 - (size_t)(unsigned)b * (unsigned)(d.H * d.W - d.bg_stride);
         if (MODE == 0 && CT == 3 && whole) {
-            const float2* src = reinterpret_cast<const float2*>(background);
+            const float2* src = reinterpret_cast<const float2*>(background + l00 * 3);
             float2* dst = reinterpret_cast<float2*>(pixels);
             float2 v[6];
 #pragma unroll
             for (int i = 0; i < 2; ++i) {
-                const size_t q = (p00 + (size_t)i * d.W) * 3 / 2;
+                const size_t q = (size_t)i * d.W * 3 / 2;   // W is even
                 v[3 * i] = __ldg(src + q); v[3 * i + 1] = __ldg(src + q + 1); v[3 * i + 2] = __ldg(src + q + 2);
             }
 #pragma unroll
@@ -388,14 +393,14 @@ __global__ void __launch_bounds__(WARPS_PER_BLOCK * 32, DIRT_RASTER_MIN_BLOCKS) 
 #pragma unroll
         for (int pix = 0; pix < 4; ++pix) {
             if (!whole && (row0 + (pix >> 1) >= d.H || col0 + (pix & 1) >= d.W)) continue;
-            const size_t p = p00 + (size_t)(pix >> 1) * d.W + (pix & 1);
+            const size_t o = (size_t)(pix >> 1) * d.W + (pix & 1), p = p00 + o;
             if (face_ids_out) face_ids_out[p] = -1;
             if (MODE == 1) {
                 if (gbuffer_out) reinterpret_cast<float4*>(gbuffer_out)[p] = make_float4(-1.f, -1.f, -1.f, __int_as_float(0x7f800000));
             } else if (CT == 4) {
-                reinterpret_cast<float4*>(pixels)[p] = __ldg(reinterpret_cast<const float4*>(background) + p);
+                reinterpret_cast<float4*>(pixels)[p] = __ldg(reinterpret_cast<const float4*>(background) + l00 + o);
             } else {
-                for (int ch = 0; ch < C; ++ch) pixels[p * C + ch] = __ldg(&background[p * C + ch]);
+                for (int ch = 0; ch < C; ++ch) pixels[p * C + ch] = __ldg(&background[(l00 + o) * C + ch]);
             }
         }
         continue;
@@ -428,7 +433,7 @@ __global__ void __launch_bounds__(WARPS_PER_BLOCK * 32, DIRT_RASTER_MIN_BLOCKS) 
         }
     }
 
-    const float* cols = vertex_colors + (size_t)b * d.V * C;
+    const float* cols = vertex_colors + (size_t)b * d.col_stride * C;
     int prev_face = -1;
     TriInterp ti;
 #pragma unroll
@@ -446,10 +451,11 @@ __global__ void __launch_bounds__(WARPS_PER_BLOCK * 32, DIRT_RASTER_MIN_BLOCKS) 
                 reinterpret_cast<float4*>(gbuffer_out)[p] = g;
             }
         } else if (face < 0) {
+            const float* bg = background + (p - (size_t)b * (d.H * d.W - d.bg_stride)) * C;   // as l00 above
             if (CT == 4) {
-                reinterpret_cast<float4*>(pixels)[p] = __ldg(reinterpret_cast<const float4*>(background) + p);
+                reinterpret_cast<float4*>(pixels)[p] = __ldg(reinterpret_cast<const float4*>(bg));
             } else {
-                for (int ch = 0; ch < C; ++ch) pixels[p * C + ch] = __ldg(&background[p * C + ch]);
+                for (int ch = 0; ch < C; ++ch) pixels[p * C + ch] = __ldg(&bg[ch]);
             }
         } else if (REC) {
             shade_pixel_record<CT>(ws.shade + (size_t)b * d.F + face, col, row, pixels + p * C, C);

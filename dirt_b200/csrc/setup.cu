@@ -30,7 +30,7 @@ __global__ void __launch_bounds__(DIRT_SETUP_THREADS, DIRT_SETUP_MIN_BLOCKS) set
 {
     const long long gid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     const long long total = (long long)d.B * d.F;
-    if (gid == 0) ws.header->tag = workspace_tag(vertices, faces, d.B, d.H, d.W, d.V, d.F);
+    if (gid == 0) ws.header->tag = workspace_tag(vertices, faces, d.B, d.H, d.W, d.V, d.F, d.face_stride == 0);
     if (gid >= total) return;
     const int b = (int)(gid / d.F);
     const int f = (int)(gid - (long long)b * d.F);
@@ -56,7 +56,7 @@ __global__ void __launch_bounds__(DIRT_SETUP_THREADS, DIRT_SETUP_MIN_BLOCKS) set
 
     int32_t vid[3];
 #pragma unroll
-    for (int k = 0; k < 3; ++k) vid[k] = __ldg(&faces[(size_t)gid * 3 + k]);
+    for (int k = 0; k < 3; ++k) vid[k] = __ldg(&faces[((size_t)b * d.face_stride + f) * 3 + k]);
     if ((unsigned)vid[0] >= (unsigned)d.V || (unsigned)vid[1] >= (unsigned)d.V || (unsigned)vid[2] >= (unsigned)d.V) { cull(); return; }
 
     float p[3][4];
@@ -144,7 +144,7 @@ __global__ void __launch_bounds__(DIRT_SETUP_THREADS, DIRT_SETUP_MIN_BLOCKS) set
         dstx[1] = make_float4(p[2][0], p[2][1], 0.f, 0.f);
         // shading record: planes of N_c = q0*(c0 - c2) + q1*(c1 - c2) + S*c2 (q2 = S - q0 - q1), values only
         if (BIN && vertex_colors != nullptr) {
-            const float* cols = vertex_colors + (size_t)b * d.V * d.C;
+            const float* cols = vertex_colors + (size_t)b * d.col_stride * d.C;
             float4 out[4];
             out[0] = make_float4(itp.sA, itp.sB, itp.sC, __uint_as_float((uint32_t)cref | ((uint32_t)rref << 16)));
             float n[12];

@@ -77,18 +77,19 @@ def _check_shapes(op, background, vertices, vertex_colors, faces, height, width,
         raise ValueError('%s expects all arguments to have same leading (batch) dimension' % op)
 
 
-def rasterise_forward_raw(background, vertices, vertex_colors, faces, want_face_ids=True, return_workspace=False):
-    """One call of dirt_rasterise_forward on contiguous CUDA tensors. Returns (pixels, face_ids or None)
-    [, workspace tensor holding the per-face setup records, reusable by rasterise_backward_raw]."""
-    B, H, W, C = background.shape
-    V, F = vertices.shape[1], faces.shape[1]
-    pixels = torch.empty_like(background)
+def rasterise_forward_raw(background, vertices, vertex_colors, faces, want_face_ids=True, return_workspace=False, shared=0):
+    """One call of dirt_rasterise_forward_ex on contiguous CUDA tensors. Returns (pixels, face_ids or None)
+    [, workspace tensor holding the per-face setup records, reusable by rasterise_backward_raw].
+    `shared`: _lib.SHARED_* bits; a shared background / vertex_colors / faces has no batch dimension."""
+    B, V, F = vertices.shape[0], vertices.shape[1], faces.shape[-2]
+    H, W, C = background.shape[-3:]
+    pixels = torch.empty((B, H, W, C), dtype=background.dtype, device=background.device)
     face_ids = torch.empty((B, H, W), dtype=torch.int32, device=background.device) if want_face_ids else None
     ws, nbytes = _workspace(B, H, W, C, V, F, background.device)
     with torch.cuda.device(background.device):
-        rc = _lib.lib().dirt_rasterise_forward(_ptr(background), _ptr(vertices), _ptr(vertex_colors), _ptr(faces),
-                                               _ptr(pixels), _ptr(face_ids), B, H, W, C, V, F, _ptr(ws), nbytes,
-                                               _stream_ptr(background.device))
+        rc = _lib.lib().dirt_rasterise_forward_ex(_ptr(background), _ptr(vertices), _ptr(vertex_colors), _ptr(faces),
+                                                  _ptr(pixels), _ptr(face_ids), B, H, W, C, V, F, _ptr(ws), nbytes,
+                                                  _stream_ptr(background.device), shared)
     _lib.check(rc, 'Rasterise')
     if return_workspace:
         ws._dirt_setup_of = _geometry_identity(vertices, faces, H, W)
@@ -103,30 +104,38 @@ def _geometry_identity(vertices, faces, H, W):
 
 
 def rasterise_backward_raw(vertices, faces, pixels, grad_pixels, face_ids=None, channel_groups=None, setup_workspace=None,
-                           shared_geometry=False, want_position=True, want_colour=True):
+                           shared_geometry=False, want_position=True, want_colour=True, shared=0, want_background=True):
     """One call of dirt_rasterise_backward (the RasteriseGrad op, csrc/rasterise_grad_egl.cpp:33-53).
     `setup_workspace`: the workspace tensor of the forward call on the same (vertices, faces); its setup records are
     reused only if it still describes exactly these tensors (storage, version counters, sizes), otherwise they are
     recomputed.  `shared_geometry`: accumulate the vertex gradients over the batch (DIRT_BWD_SHARED_GEOMETRY):
     grad_vertices [V,4] and grad_vertex_colors [V,C] instead of [B,V,.].  want_position / want_colour = False skip
     the position terms (grad_vertices comes back zero) / the colour terms (grad_vertex_colors zero, grad_background None).
+    `shared`: the _lib.SHARED_* bits of the forward call.  A shared background's gradient is [H,W,C], summed over the batch,
+    and is computed only when `want_background`; shared colours get a [V,C] gradient, summed over the batch; shared faces
+    are [F,3].
     Returns (grad_background, grad_vertices, grad_vertex_colors)."""
     B, H, W, C = pixels.shape
-    V, F = vertices.shape[1], faces.shape[1]
+    V, F = vertices.shape[1], faces.shape[-2]
+    faces_rank = 2 if shared & _lib.SHARED_FACES else 3
     # wording of csrc/rasterise_grad_egl.cpp:349-377
     if vertices.dim() != 3 or vertices.shape[2] != 4:
         raise ValueError('RasteriseGrad expects vertices to be 3D, and vertices.shape[2] == 4')
-    if faces.dim() != 3 or faces.shape[2] != 3:
-        raise ValueError('RasteriseGrad expects faces to be 3D, and faces.shape[2] == 3')
+    if faces.dim() != faces_rank or faces.shape[-1] != 3:
+        raise ValueError('RasteriseGrad expects faces to be %dD, and faces.shape[%d] == 3' % (faces_rank, faces_rank - 1))
     if grad_pixels.shape != pixels.shape:
         raise ValueError('RasteriseGrad expects grad_pixels to be 4D, and grad_pixels.shape == [None, height, width, channels]')
-    if faces.shape[0] != B or vertices.shape[0] != B:
+    if (faces_rank == 3 and faces.shape[0] != B) or vertices.shape[0] != B:
         raise ValueError('RasteriseGrad expects all arguments to have same leading (batch) dimension')
     device = pixels.device
-    grad_background = torch.empty_like(pixels) if want_colour else None
+    if shared & _lib.SHARED_BACKGROUND:
+        grad_background = torch.empty((H, W, C), dtype=torch.float32, device=device) if want_colour and want_background else None
+    else:
+        grad_background = torch.empty_like(pixels) if want_colour else None
     lead = () if shared_geometry else (B,)
     grad_vertices = torch.empty(lead + (V, 4), dtype=torch.float32, device=device)
-    grad_vertex_colors = torch.empty(lead + (V, C), dtype=torch.float32, device=device)
+    colour_lead = () if shared & _lib.SHARED_COLOURS else lead
+    grad_vertex_colors = torch.empty(colour_lead + (V, C), dtype=torch.float32, device=device)
     if channel_groups is None:
         groups_ptr, n_groups = None, 0
     else:
@@ -138,7 +147,7 @@ def rasterise_backward_raw(vertices, faces, pixels, grad_pixels, face_ids=None, 
     ws = setup_workspace if reuse else _workspace(B, H, W, C, V, F, device, face_id_scratch=face_ids is None)[0]
     nbytes = int(ws.numel())
     flags = ((_lib.BWD_SHARED_GEOMETRY if shared_geometry else 0) | (0 if want_position else _lib.BWD_SKIP_POSITION) |
-             (0 if want_colour else _lib.BWD_SKIP_COLOUR))
+             (0 if want_colour else _lib.BWD_SKIP_COLOUR) | shared)
     with torch.cuda.device(device):
         rc = _lib.lib().dirt_rasterise_backward_ex(
             _ptr(vertices), _ptr(faces), _ptr(pixels), _ptr(grad_pixels), _ptr(face_ids),
@@ -172,15 +181,17 @@ def rasterise_visibility_raw(vertices, faces, height, width, want_gbuffer=True):
 
 
 class _Rasterise(torch.autograd.Function):
-    """The Rasterise op with its registered gradient (dirt/rasterise_ops.py:111-129)."""
+    """The Rasterise op with its registered gradient (dirt/rasterise_ops.py:111-129).  `shared`: _lib.SHARED_* bits of the
+    inputs the whole batch shares (0: every input per image)."""
 
     @staticmethod
-    def forward(ctx, background, vertices, vertex_colors, faces, channel_groups):
+    def forward(ctx, background, vertices, vertex_colors, faces, channel_groups, shared=0):
         pixels, face_ids, ws = rasterise_forward_raw(background, vertices, vertex_colors, faces, want_face_ids=True,
-                                                     return_workspace=True)
+                                                     return_workspace=True, shared=shared)
         ctx.save_for_backward(vertices, faces, pixels, face_ids)
         ctx.setup_workspace = ws   # per-face setup records of this (vertices, faces): backward reuses them
         ctx.channel_groups = channel_groups
+        ctx.shared = shared
         ctx.mark_non_differentiable(face_ids)
         return pixels, face_ids
 
@@ -188,14 +199,16 @@ class _Rasterise(torch.autograd.Function):
     def backward(ctx, grad_pixels, _grad_face_ids):
         want_background, want_vertices, want_colours = ctx.needs_input_grad[:3]
         if not (want_background or want_vertices or want_colours):
-            return None, None, None, None, None
+            return None, None, None, None, None, None
         vertices, faces, pixels, face_ids = ctx.saved_tensors
         grad_pixels = grad_pixels.contiguous().to(torch.float32)
+        # a shared background that needs no gradient gets none: no per-image gradient is written and nothing is summed
         grad_background, grad_vertices, grad_vertex_colors = rasterise_backward_raw(
             vertices, faces, pixels, grad_pixels, face_ids, ctx.channel_groups, ctx.setup_workspace,
-            want_position=want_vertices, want_colour=want_background or want_colours)
+            want_position=want_vertices, want_colour=want_background or want_colours, shared=ctx.shared,
+            want_background=want_background)
         return (grad_background if want_background else None, grad_vertices if want_vertices else None,
-                grad_vertex_colors if want_colours else None, None, None)  # None: wrt faces
+                grad_vertex_colors if want_colours else None, None, None, None)  # None: wrt faces
 
 
 def _as_f32(x, device=None):
@@ -272,6 +285,48 @@ def rasterise_batch(background, vertices, vertex_colors, faces, height=None, wid
     groups = default_channel_groups(channels)
     pixels, _ = _Rasterise.apply(background.contiguous(), vertices.contiguous(), vertex_colors.contiguous(),
                                  faces.contiguous(), groups)
+    return pixels
+
+
+def rasterise_batch_shared(background, vertices, vertex_colors, faces, height=None, width=None, channels=None, name=None):
+    """`rasterise_batch` for one mesh in B poses: only `vertices` [B,V,4] must carry the batch dimension.
+
+    `background` is [B,H,W,C] or [H,W,C], `vertex_colors` [B,V,C] or [V,C], `faces` [B,F,3] or [F,3]: the rank of each
+    decides whether it is per image or shared by the whole batch.  The pixels equal `rasterise_batch` called with the
+    shared arguments expanded to B, without B copies of them; the gradient of a shared argument has that argument's own
+    shape and is the sum of the per-image gradients over the batch (a shared background's gradient is only computed when
+    the background requires grad).
+    """
+    device = _pick_device(background, vertices, vertex_colors, faces)
+    background = _as_f32(background, device)
+    vertices = _as_f32(vertices, device)
+    vertex_colors = _as_f32(vertex_colors, device)
+    faces = _as_i32(faces, device)
+    if vertices.dim() != 3 or vertices.shape[2] != 4:
+        raise ValueError('Rasterise expects vertices to be 3D, and vertices.shape[2] == 4')
+    if background.dim() not in (3, 4):
+        raise ValueError('Rasterise expects background_tensor to be 4D, and bgcolor.shape == [None, height, width, channels]')
+    B = int(vertices.shape[0])
+    shared = ((_lib.SHARED_BACKGROUND if background.dim() == 3 else 0) | (_lib.SHARED_COLOURS if vertex_colors.dim() == 2 else 0) |
+              (_lib.SHARED_FACES if faces.dim() == 2 else 0))
+    if height is None:
+        height = int(background.shape[-3])
+    if width is None:
+        width = int(background.shape[-2])
+    if channels is None:
+        channels = int(background.shape[-1])
+    if not (channels > 0):
+        raise ValueError('channels must be positive')
+    if not (width > 0 and height > 0):
+        raise ValueError('width and height must be positive')
+    # the checks (and messages) of rasterise_batch on batch-dimensioned views of the shared arguments (no copies)
+    batched = lambda t, bit: t.expand((B,) + tuple(t.shape)) if shared & bit else t
+    _check_shapes('Rasterise', batched(background, _lib.SHARED_BACKGROUND), vertices, batched(vertex_colors, _lib.SHARED_COLOURS),
+                  batched(faces, _lib.SHARED_FACES), height, width, channels)
+    _require_cuda(background, vertices, vertex_colors, faces)
+    groups = default_channel_groups(channels)
+    pixels, _ = _Rasterise.apply(background.contiguous(), vertices.contiguous(), vertex_colors.contiguous(), faces.contiguous(),
+                                 groups, shared)
     return pixels
 
 

@@ -25,6 +25,7 @@
  *   vertex_colors, grad_vertex_colors                : float32 [B, V, C]
  *   faces                                            : int32   [B, F, 3]
  *   face_ids                                         : int32   [B, H, W]   (-1 = background)
+ * except for an input the whole batch shares (DIRT_SHARED_* below), which has no batch dimension.
  *   gbuffer                                          : float32 [B, H, W, 4] (bary0, bary1, bary2, clip_w;
  *                                                      (-1,-1,-1,+inf) where uncovered)
  */
@@ -78,6 +79,28 @@ int dirt_rasterise_forward(const float* background, const float* vertices,
                            int B, int H, int W, int C, int V, int F,
                            void* workspace, size_t workspace_bytes, void* cuda_stream);
 
+/* Inputs the whole batch shares (one mesh in B poses): a shared tensor has no batch dimension.  The values do not collide
+ * with the DIRT_BWD_* bits, so one flags word serves a forward and its backward call.
+ *  DIRT_SHARED_BACKGROUND  background is [H,W,C]; in a backward call grad_background is [H,W,C], the sum over the batch of
+ *                          the per-image gradients, or NULL when it is not wanted (then nothing is computed for it).
+ *  DIRT_SHARED_COLOURS     vertex_colors is [V,C]; in a backward call grad_vertex_colors is [V,C], summed over the batch
+ *                          (grad_vertices stays [B,V,4] unless DIRT_BWD_SHARED_GEOMETRY is also set).
+ *  DIRT_SHARED_FACES       faces is [F,3].  The setup records stay per image (the vertices are), and the workspace tag
+ *                          includes the face layout, so a workspace_holds_setup promise across layouts is caught. */
+enum {
+    DIRT_SHARED_BACKGROUND = 8,
+    DIRT_SHARED_COLOURS = 16,
+    DIRT_SHARED_FACES = 32
+};
+
+/* dirt_rasterise_forward with a flags word (flags = 0 is dirt_rasterise_forward itself); only the DIRT_SHARED_* bits are
+ * accepted. */
+int dirt_rasterise_forward_ex(const float* background, const float* vertices,
+                              const float* vertex_colors, const int32_t* faces,
+                              float* pixels, int32_t* face_ids_out,
+                              int B, int H, int W, int C, int V, int F,
+                              void* workspace, size_t workspace_bytes, void* cuda_stream, int flags);
+
 /* Backward: the RasteriseGrad op.  `pixels` is an input (deferred shading passes shaded
  * pixels, rasterise_ops.py:206-210).  channel_groups (host pointer) lists the widths of the
  * reference's channel groups, e.g. {3,1} for C=4; each group takes its own Scharr / dilation
@@ -110,7 +133,8 @@ int dirt_rasterise_backward(const float* vertices, const int32_t* faces,
  *  DIRT_BWD_SKIP_POSITION    grad_vertices is not computed (left zero): no Scharr filter, no dilation, `pixels` is not read.
  *  DIRT_BWD_SKIP_COLOUR      grad_vertex_colors is not computed (left zero) and grad_background is not written.
  *  The two SKIP flags serve deferred shading, whose gradient is two RasteriseGrad calls of which only one output each
- *  is used (dirt/rasterise_ops.py:206-237: vertices from the shaded pixels, attributes / background from the G-buffer). */
+ *  is used (dirt/rasterise_ops.py:206-237: vertices from the shaded pixels, attributes / background from the G-buffer).
+ *  The DIRT_SHARED_* bits of dirt_rasterise_forward_ex are accepted as well. */
 enum {
     DIRT_BWD_SHARED_GEOMETRY = 1,
     DIRT_BWD_SKIP_POSITION = 2,
@@ -158,7 +182,8 @@ int dirt_last_launch_count(void);
  * csrc/rasterise_egl.cpp:284-286,398-405): bracket ONE kernel of subsequent calls on this thread with
  * CUDA events recorded on the call's own stream.  which: 0 = off, 1 = forward raster kernel,
  * 2 = backward (assemble-grads) kernel.  dirt_kernel_timer_elapsed_ms() waits for the last bracketed
- * launch and returns its duration in milliseconds (negative if nothing was timed). */
+ * launch and returns its duration in milliseconds (negative if nothing was timed).  which = 3: the kernel that sums a
+ * shared background's gradient over the batch (DIRT_SHARED_BACKGROUND). */
 int dirt_kernel_timer_enable(int which);
 float dirt_kernel_timer_elapsed_ms(void);
 
